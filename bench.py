@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- particle-steps/s of the SPHSystem::step() hot path on a synthetic dam-break.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload dfsph|wcsph|pbd] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload dfsph|wcsph|pbd] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one SPHSystem::step(): neighbour search + one solver step over the whole particle set.
 Default workload at N=1: BASELINE.json configs[2], the configuration the north-star target is quoted on
@@ -28,6 +28,9 @@ driven through the very same facade source -- the "reference build" of the north
 scene, timed as the median of per-step wall times (its own cudaEvent figure is reported beside it); if that
 library is absent, the CPU restatement is timed instead (kind "port").
 N>1: every line is self-checked first (slabs.parity_check: two steps against a single-GPU run of the same scene).
+--dump-outputs DIR (N=1): after the timed steps, the fluid state the timed path left after its last step is written as
+DIR/{pos,vel,density,pressure}.npy (float32, rows in the engine's sorted order; see dump_outputs).  The scenes are
+deterministic lattices, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -57,6 +60,22 @@ ALG_BYTES = {  # SURVEY.md section 8(d): algorithmic HBM bytes per fluid particl
     "pbd_xsph+color_grad": 52,        # xsph 40 + colour gradient 28 - shared pos/mass 16
 }
 SCENE_OF_N = {1: "2m", 2: "4m", 4: "8m", 8: "16m"}
+DUMP_FIELDS = ("pos", "vel", "density", "pressure")
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir: str, state: dict, seed: int = 0) -> None:
+    """Writes state[f] for f in DUMP_FIELDS as out_dir/<f>.npy (float32).  When all rows together would exceed
+    DUMP_BYTES, every array keeps the same rows: a sample drawn with a fixed seed, in increasing row order."""
+    arrays = {f: np.ascontiguousarray(state[f], np.float32) for f in DUMP_FIELDS}
+    n = arrays["pos"].shape[0]
+    keep = min(n, (DUMP_BYTES - 4096) // (sum(a.nbytes for a in arrays.values()) // n))   # 4096: the .npy headers
+    if keep < n:
+        rows = np.sort(np.random.default_rng(seed).choice(n, size=keep, replace=False))
+        arrays = {f: a[rows] for f, a in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for f, a in arrays.items():
+        np.save(os.path.join(out_dir, f + ".npy"), a)
 
 
 def peaks():
@@ -193,7 +212,7 @@ def run_reference(args, pkg) -> dict:
     n = sc.fluid.shape[0]
     app = capi.SphApp(sc, libref)
     warm = max(args.warmup, 5)
-    steps = max(args.steps, 20)
+    steps = args.steps
     for _ in range(warm):
         app.step()
     # Estimator: the MEDIAN of per-step host wall times (SPHSystem::step() synchronises the device before it returns,
@@ -210,6 +229,8 @@ def run_reference(args, pkg) -> dict:
         wall.append(time.perf_counter() - t0)
     torch.cuda.synchronize()
     t_all = time.perf_counter() - t_all
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, app.download())
     sampler = ClockSampler(0, period_ms=500); sampler.start()
     for _ in range(steps):
         app.step()
@@ -322,6 +343,8 @@ def run_ours_single(args, pkg) -> dict:
     ms_total = e_start.elapsed_time(e_stop)
     clocks = sampler.stop()
     launches = s.launch_count() - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, s.state())
     ms_step = ms_total / args.steps
     value = n / (ms_step * 1e-3)
     peak, peak_src = peaks()
@@ -419,11 +442,17 @@ def main():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak (default, the driver's contract): 2M fluid particles per GPU, N=8 is BASELINE configs[4]; "
                          "strong: the same scene (--scene, default 2m) split over N GPUs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the state after the last timed step as DIR/<name>.npy (single-GPU runs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     args.warmup = max(args.warmup, 3)
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (world > 1 or args.gpus > 1) and args.impl == "ours":
+        ap.error("--dump-outputs writes the single-GPU path's outputs: use it with --gpus 1")
     import pkgload
     pkg = pkgload.load()
-    world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
         out = run_reference(args, pkg)
         if out:

@@ -1,9 +1,9 @@
 """Whole-step parity on the GPU:
   * the C++ class layer (libsphhost.so, through the reference's own call sites restated in sph_app.cpp)
-    against the reference's own CUDA kernels (oracle/_ref/libsphref.so = the unmodified reference .cu
-    files compiled for sm_100) on identical inputs: bit-exact particle2cell / sort order / cellStart,
-    <= 1e-5 scale-relative on positions and densities after the constructor (step 0, Q3) and after each
-    explicit step;
+    against the reference's own CUDA kernels (the unmodified reference .cu files compiled for sm_100, run on a
+    B200 by tests/golden/make_golden.py, outputs stored in tests/golden/reference_cuda.npz) on identical inputs:
+    bit-exact particle2cell / sort order / cellStart (sha256 over all particles), <= 1e-5 scale-relative on
+    positions and densities after the constructor (step 0, Q3) and after each explicit step (on stored rows);
   * the same against the CPU restatement (oracle/) and against the committed golden fixtures;
   * the python mirror (engine.SphkSystem) against the C++ layer (must be identical: same C-ABI calls).
 """
@@ -12,7 +12,7 @@ import os
 import numpy as np
 import pytest
 
-from util import GOLDEN, LIBREF, TOL, assert_close, bits, cell_start_from_p2c, relerr
+from util import GOLDEN, TOL, assert_close, assert_close_sample, bits, cell_start_from_p2c, digest, relerr
 
 pytestmark = pytest.mark.gpu
 
@@ -25,6 +25,17 @@ def _gpu():
         pytest.fail("pytest -m gpu needs a CUDA device: libsphk has no CPU fallback")
 
 
+@pytest.fixture(scope="module")
+def gold():
+    """Outputs of the reference's own CUDA kernels (tests/golden/make_golden.py)."""
+    with np.load(os.path.join(GOLDEN, "reference_cuda.npz")) as z:
+        return {k: z[k] for k in z.files}
+
+
+def _same_bits(a, gold, key):
+    return digest(a) == str(gold[key + ".sha256"])
+
+
 def _run(app, steps):
     out = [app.download()]
     for _ in range(steps):
@@ -33,109 +44,106 @@ def _run(app, steps):
     return out
 
 
-def _compare_states(ours, ref, what, vel_tol=2e-4):
-    assert np.array_equal(ours["p2c"], ref["p2c"]), f"{what}: particle2cell differs"
-    assert_close(ours["pos"], ref["pos"], what=f"{what} pos")
-    assert_close(ours["density"], ref["density"], what=f"{what} density")
-    assert_close(ours["vel"], ref["vel"], tol=vel_tol, what=f"{what} vel")
-    assert_close(ours["pressure"], ref["pressure"], tol=1e-4, what=f"{what} pressure")
+def _compare_states(ours, gold, key, what, vel_tol=2e-4):
+    assert _same_bits(ours["p2c"], gold, key + ".p2c"), f"{what}: particle2cell differs"
+    assert_close_sample(ours["pos"], gold, key + ".pos", what=f"{what} pos")
+    assert_close_sample(ours["density"], gold, key + ".density", what=f"{what} density")
+    assert_close_sample(ours["vel"], gold, key + ".vel", tol=vel_tol, what=f"{what} vel")
+    assert_close_sample(ours["pressure"], gold, key + ".pressure", tol=1e-4, what=f"{what} pressure")
+
+
+def _compare_boundary(app, gold, case):
+    b, key = app.download_boundary(), case + "-boundary"
+    assert _same_bits(b["p2c"], gold, key + ".p2c")
+    assert _same_bits(b["pos"], gold, key + ".pos"), "sorted boundary positions must be bit-identical"
+    assert_close_sample(b["mass"], gold, key + ".mass", what=f"{case} boundary mass")
 
 
 @pytest.mark.parametrize("solver", SOLVERS)
 @pytest.mark.parametrize("name,jitter", [("config0", 0.0), ("config0", 0.001)])
-def test_class_layer_vs_reference_cuda(pkg, built, solver, name, jitter):
+def test_class_layer_vs_reference_cuda(pkg, built, gold, solver, name, jitter):
     _gpu()
-    if not os.path.exists(LIBREF):
-        pytest.skip("oracle/_ref/libsphref.so not built (reference sources absent at build time)")
     from cpp_fluid_particles_b200 import capi
     sc = pkg.scene.benchmark_scene(name, solver)
     if jitter:
         sc = pkg.scene.make_scene(name, solver=solver, dt=sc.params.dt, max_iter=sc.params.max_iter,
                                   den_thr=sc.params.density_error_threshold, div_thr=sc.params.divergence_error_threshold,
                                   jitter=jitter)
+    case = f"{name}{'-jitter' if jitter else ''}-{solver}"
     ours_app = capi.SphApp(sc)
-    ref_app = capi.SphApp(sc, LIBREF)
-    assert ours_app.engine == "b200-native" and ref_app.engine == "reference-cuda"
-    ours, ref = _run(ours_app, 3), _run(ref_app, 3)
+    assert ours_app.engine == "b200-native"
+    ours = _run(ours_app, 3)
     # boundary set: searched once in the constructor
-    ob, rb = ours_app.download_boundary(), ref_app.download_boundary()
-    assert np.array_equal(ob["p2c"], rb["p2c"])
-    assert np.array_equal(bits(ob["pos"]), bits(rb["pos"])), "sorted boundary positions must be bit-identical"
-    assert_close(ob["mass"], rb["mass"], what="boundary mass")
-    for k, (o, r) in enumerate(zip(ours, ref)):
+    _compare_boundary(ours_app, gold, case)
+    for k, o in enumerate(ours):
         if solver == "pbd" and k == 0:
             # Q6: PBD's step 0 is neighbour search + posLast init only -> pure sort: bit-identical order
-            assert np.array_equal(bits(o["pos"]), bits(r["pos"])), "sort permutation differs from the reference"
-        _compare_states(o, r, f"{solver} after step {k}")
-    ours_app.close(); ref_app.close()
+            assert _same_bits(o["pos"], gold, f"{case}.s0.pos"), "sort permutation differs from the reference"
+        _compare_states(o, gold, f"{case}.s{k}", f"{solver} after step {k}")
+    ours_app.close()
 
 
-def test_class_layer_vs_reference_cuda_200k(pkg, built):
+def test_class_layer_vs_reference_cuda_200k(pkg, built, gold):
     """A denser check at 216 000 fluid + 58 808 boundary particles (DFSPH 4+4): two steps against the reference's
     own kernels."""
     _gpu()
-    if not os.path.exists(LIBREF):
-        pytest.skip("oracle/_ref/libsphref.so not built")
     from cpp_fluid_particles_b200 import capi
     sc = pkg.scene.benchmark_scene("200k", "dfsph")
-    a, b = capi.SphApp(sc), capi.SphApp(sc, LIBREF)
+    a = capi.SphApp(sc)
     for k in range(3):
-        _compare_states(a.download(), b.download(), f"200k dfsph step {k}")
-        a.step(); b.step()
-    a.close(); b.close()
+        _compare_states(a.download(), gold, f"200k-dfsph.s{k}", f"200k dfsph step {k}")
+        a.step()
+    a.close()
 
 
 @pytest.mark.parametrize("solver", SOLVERS)
-def test_class_layer_vs_reference_cuda_2m(pkg, built, solver):
+def test_class_layer_vs_reference_cuda_2m(pkg, built, gold, solver):
     """BASELINE.json configs[1-3] at their real size (2 097 152 fluid + 237 608 boundary particles): the C++ class
     layer against the reference's own CUDA kernels -- constructor state (step 0, Q3) and one explicit step.
     Bit-exact particle2cell / cellStart / sorted boundary; <= 1e-5 scale-relative on positions and densities, and
-    <= 1e-5 PER ELEMENT on the densities of interior particles (rho >= 0.9 rho0: no free-surface cancellation)."""
+    <= 1e-5 PER ELEMENT on the densities of interior particles (rho >= 0.9 rho0: no free-surface cancellation) among
+    the stored rows."""
     _gpu()
-    if not os.path.exists(LIBREF):
-        pytest.skip("oracle/_ref/libsphref.so not built")
     from cpp_fluid_particles_b200 import capi
     sc = pkg.scene.benchmark_scene("2m", solver)
-    a, b = capi.SphApp(sc), capi.SphApp(sc, LIBREF)
-    ob, rb = a.download_boundary(), b.download_boundary()
-    assert np.array_equal(ob["p2c"], rb["p2c"])
-    assert np.array_equal(bits(ob["pos"]), bits(rb["pos"]))
-    assert_close(ob["mass"], rb["mass"], what="2m boundary mass")
+    case = f"2m-{solver}"
+    a = capi.SphApp(sc)
+    _compare_boundary(a, gold, case)
     nc = sc.params.ncells
+    idx = gold[case + ".idx"]
     for k in range(2):
-        sa, sb = a.download(), b.download()
-        assert np.array_equal(sa["p2c"], sb["p2c"]), f"2m {solver} step {k}: particle2cell differs"
-        assert np.array_equal(cell_start_from_p2c(sa["p2c"], nc), cell_start_from_p2c(sb["p2c"], nc))
-        assert_close(sa["pos"], sb["pos"], what=f"2m {solver} step {k} pos")
-        assert_close(sa["density"], sb["density"], what=f"2m {solver} step {k} density")
+        sa, key = a.download(), f"{case}.s{k}"
+        assert _same_bits(sa["p2c"], gold, key + ".p2c"), f"2m {solver} step {k}: particle2cell differs"
+        assert _same_bits(cell_start_from_p2c(sa["p2c"], nc), gold, key + ".cell_start")
+        assert_close_sample(sa["pos"], gold, key + ".pos", what=f"2m {solver} step {k} pos")
+        assert_close_sample(sa["density"], gold, key + ".density", what=f"2m {solver} step {k} density")
         if solver == "pbd" and k == 0:
-            assert np.array_equal(bits(sa["pos"]), bits(sb["pos"])), "sort permutation differs from the reference"
-        interior = sb["density"] >= 0.9 * sc.params.rho0
+            assert _same_bits(sa["pos"], gold, key + ".pos"), "sort permutation differs from the reference"
+        ref_d = gold[key + ".density"]
+        interior = ref_d >= 0.9 * sc.params.rho0
         if interior.any():
-            d = np.abs(sa["density"][interior].astype(np.float64) - sb["density"][interior]) / sb["density"][interior]
+            d = np.abs(sa["density"][idx][interior].astype(np.float64) - ref_d[interior]) / ref_d[interior]
             assert d.max() <= 1e-5, f"2m {solver} step {k}: per-element interior density error {d.max():.2e}"
-        a.step(); b.step()
-    a.close(); b.close()
+        a.step()
+    a.close()
 
 
 @pytest.mark.parametrize("solver", SOLVERS)
-def test_sorted_order_bit_exact_through_steps(pkg, built, solver):
+def test_sorted_order_bit_exact_through_steps(pkg, built, gold, solver):
     """The stable-sort permutation and cellStart stay identical to the reference while the fluid moves:
     particle2cell of step k is computed from positions that already differ by ~1e-7, so exact equality of
     the keys over several steps is a strong check of both the physics and the hash."""
     _gpu()
-    if not os.path.exists(LIBREF):
-        pytest.skip("oracle/_ref/libsphref.so not built")
     from cpp_fluid_particles_b200 import capi
     sc = pkg.scene.benchmark_scene("mini", solver)
-    a, b = capi.SphApp(sc), capi.SphApp(sc, LIBREF)
+    a = capi.SphApp(sc)
     for k in range(6):
-        a.step(); b.step()
-        sa, sb = a.download(), b.download()
-        assert np.array_equal(sa["p2c"], sb["p2c"]), f"step {k}"
+        a.step()
+        sa = a.download()
+        assert _same_bits(sa["p2c"], gold, f"mini-{solver}.s{k}.p2c"), f"step {k}"
         nc = sc.params.ncells
-        assert np.array_equal(cell_start_from_p2c(sa["p2c"], nc), cell_start_from_p2c(sb["p2c"], nc))
-    a.close(); b.close()
+        assert _same_bits(cell_start_from_p2c(sa["p2c"], nc), gold, f"mini-{solver}.s{k}.cell_start")
+    a.close()
 
 
 @pytest.mark.parametrize("solver", SOLVERS)

@@ -1,4 +1,5 @@
 """Shared helpers of the parity tests."""
+import hashlib
 import os
 
 import numpy as np
@@ -23,6 +24,20 @@ def relerr(a, b) -> float:
 def assert_close(a, b, tol=TOL, what=""):
     e = relerr(a, b)
     assert e <= tol, f"{what}: scale-relative error {e:.3e} > {tol:.1e}"
+
+
+def assert_close_sample(a, gold, key, tol=TOL, what=""):
+    """assert_close against a stored sample of a reference field: rows gold[<case>.idx] of `a` against gold[key],
+    relative to max |b| over the WHOLE reference field (gold[key + '.scale']) -- relerr's measure on the sampled rows."""
+    idx = gold[key.split(".")[0] + ".idx"]
+    d = np.abs(np.asarray(a, np.float64)[idx] - np.asarray(gold[key], np.float64))
+    e = float(np.max(d)) / max(float(gold[key + ".scale"]), 1e-30)
+    assert e <= tol, f"{what}: scale-relative error {e:.3e} > {tol:.1e} (on {idx.size} stored rows)"
+
+
+def digest(a) -> str:
+    """sha256 of an array's bytes: a bit-exact comparison with a stored reference output without storing the output."""
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
 
 
 def bits(a):
